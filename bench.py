@@ -265,6 +265,26 @@ def parity_vs_single(agent, world):
             "allreduce_ms": a.elapsed_time(b) / 10.0, "allreduce_bytes": buf.numel() * 4}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, info, model):
+    """What a caller of the timed path holds after its last step: the info dict train_epochs returned (float64 scalars,
+    info.<key>.npy) and the parameters that step left in the model (float32, param.<name>.npy; 13.4 MB at this workload)."""
+    arrays = {}
+    for k, v in info.items():
+        for kk, vv in (v.items() if isinstance(v, dict) else [("", v)]):
+            arrays["info.%s%s" % (k, "." + kk if kk else "")] = np.asarray(float(vv), np.float64)
+    for k, v in model.state_dict().items():
+        arrays["param." + k] = v.detach().float().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, "outputs to dump: %d bytes" % total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return total
+
+
 def _log(msg):
     if os.environ.get("XB_BENCH_VERBOSE", "1") != "0":
         sys.stderr.write("[bench %6.1fs rank %s] %s\n" % (time.time() - _T0, os.environ.get("RANK", "0"), msg))
@@ -354,6 +374,8 @@ def run_own_arm(args):
     barrier()
     elapsed_ms = e0.elapsed_time(e1)
     _log("timed region done: %.1f ms/step" % (elapsed_ms / args.steps))
+    if args.dump_outputs and rank == 0:      # before anything below (e2e steps) moves the weights on
+        _log("dumped %d bytes of outputs to %s" % (dump_outputs(args.dump_outputs, info, agent.model), args.dump_outputs))
     launches = _lib.launch_count - launches0
     clocks = sampler.stop() if sampler else None
     t = torch.tensor([elapsed_ms], dtype=torch.float64, device=device)
@@ -530,6 +552,9 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--graph", type=int, default=-1, help="CUDA-graph the minibatch update: 1/0; default: on (every N)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's info dict and model parameters to DIR/<name>.npy "
+                         "(inputs are seeded: the same arguments give the same inputs, so two builds can be compared)")
     args = ap.parse_args()
     if args.warmup < 3 and args.impl != "reference":
         args.warmup = 3

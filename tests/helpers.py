@@ -80,6 +80,80 @@ def qmix_episode_stream(rng, keys, n_envs, T, obs_dim, A, S, episodes):
                                              state=rng.normal(size=S).astype(np.float32)))
 
 
+def flatten(obj, path=""):
+    """Nested dict / list / tuple / ndarray / scalar -> {path: ndarray}, the form the golden .npz files store results in."""
+    out = {}
+    if isinstance(obj, dict):
+        for k in obj:
+            out.update(flatten(obj[k], "%s/%s" % (path, k)))
+    elif isinstance(obj, (list, tuple)):
+        out[path + "#len"] = np.array(len(obj))
+        for i, x in enumerate(obj):
+            out.update(flatten(x, "%s[%d]" % (path, i)))
+    else:
+        out[path] = np.asarray(obj)
+    return out
+
+
+def array_digest(a):
+    """sha256 of dtype, shape and bytes: a bit-exact stand-in for an array too large to store."""
+    import hashlib
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode() + a.tobytes()).hexdigest()
+
+
+def structure_digest(obj):
+    """sha256 over the paths, shapes and values (as float64, or text) of a nested result: equal exactly when
+    same_structure(a, b) holds for the two objects."""
+    import hashlib
+    h = hashlib.sha256()
+    for path, v in sorted(flatten(obj).items()):
+        v = v.astype(np.float64) if v.dtype.kind in "biuf" else v.astype(str)
+        h.update(("%s%s%s" % (path, v.dtype.kind, v.shape)).encode() + np.ascontiguousarray(v).tobytes())
+    return h.hexdigest()
+
+
+def state_sample_index(n, size=64):
+    """The fixed element sample of an n-element tensor that golden files keep (all of it when small)."""
+    return np.arange(n) if n <= size else np.sort(np.random.default_rng(n).choice(n, size, replace=False))
+
+
+def record_state(out, prefix, state_dict, sample=True):
+    """Stores, per tensor (in state_dict order, under /keys), float64 sum and abs-sum digests and (sample=True) a fixed element sample."""
+    out[prefix + "/keys"] = np.array(list(state_dict), dtype=str)
+    flats = [v.detach().reshape(-1).numpy().astype(np.float64) for v in state_dict.values()]
+    out[prefix + "/digest"] = np.array([[f.sum(), np.abs(f).sum()] for f in flats])
+    if sample:
+        out[prefix + "/val"] = np.concatenate([f[state_sample_index(f.size)] for f in flats]).astype(np.float32)
+
+
+def assert_state_close(state_dict, g, prefix, rtol, atol):
+    """Elementwise allclose on the recorded sample; the abs-sum over ALL elements within the bound elementwise closeness
+    implies (n * atol + rtol * sum|expected|)."""
+    keys = list(g[prefix + "/keys"])
+    assert sorted(state_dict) == sorted(keys), (sorted(state_dict), sorted(keys))
+    pos = 0
+    for k, (_, ref_abs) in zip(keys, g[prefix + "/digest"]):
+        flat = state_dict[k].detach().reshape(-1).cpu().numpy()
+        idx = state_sample_index(flat.size)
+        np.testing.assert_allclose(flat[idx], g[prefix + "/val"][pos:pos + idx.size], rtol=rtol, atol=atol, err_msg=k)
+        pos += idx.size
+        got_abs = np.abs(flat.astype(np.float64)).sum()
+        assert abs(got_abs - ref_abs) <= flat.size * atol + rtol * ref_abs, (k, got_abs, ref_abs)
+
+
+def assert_same_init(state_dict, g, prefix):
+    """Initial weights rebuilt from the seed equal the reference's (float64 sum and abs-sum of every tensor).  rtol 1e-6:
+    torch's orthogonal_ initialiser runs a LAPACK QR whose last bits depend on the host CPU; a different construction
+    order changes the digests at order 1.  The signed sum cancels, so its tolerance is taken relative to the abs-sum."""
+    keys = list(g[prefix + "/keys"])
+    assert sorted(state_dict) == sorted(keys), (sorted(state_dict), sorted(keys))
+    for k, (ref_sum, ref_abs) in zip(keys, g[prefix + "/digest"]):
+        flat = state_dict[k].detach().reshape(-1).double()
+        np.testing.assert_allclose(flat.abs().sum().item(), ref_abs, rtol=1e-6, err_msg=k)
+        np.testing.assert_allclose(flat.sum().item(), ref_sum, rtol=0, atol=1e-6 * ref_abs, err_msg=k)
+
+
 def same_structure(a, b, path=""):
     """Structural equality of nested dict / list / ndarray / scalar results."""
     if isinstance(a, dict):

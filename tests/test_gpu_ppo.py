@@ -124,7 +124,14 @@ def test_ppo_learner_update_matches_oracle(compute, tol):
 
 @pytest.mark.parametrize("kind", ["a2c", "pg"])
 def test_a2c_pg_learners_match_oracle(kind):
-    """Sibling learners on the same K4 kernel (loss_kind = 1): A2C and PG (SURVEY.md section 8f-3)."""
+    """Sibling learners on the same K4 kernel (loss_kind = 1): A2C and PG (SURVEY.md section 8f-3).  The fp32 encoder's
+    convolutions run without cuDNN here: on B200 cuDNN's fp32 weight-gradient algorithm for conv2 is off by enough, on a
+    few PG gradient elements near Adam's eps, to move those weights by ~lr after three steps."""
+    with torch.backends.cudnn.flags(enabled=False, benchmark=False, deterministic=False, allow_tf32=False):
+        _a2c_pg_learners_match_oracle(kind)
+
+
+def _a2c_pg_learners_match_oracle(kind):
     from xuance_b200.torch.learners import A2C_Learner, PG_Learner
     from xuance_b200.common import BaseCallback
     torch.manual_seed(2)

@@ -1,167 +1,134 @@
-"""CPU, build container only (needs /root/reference): the oracle next to the LIVE, unmodified reference on fresh
-seeded inputs - the second way the oracle is pinned (the first is tests/golden).  Skipped where the reference is absent."""
+"""CPU: the oracle next to the unmodified reference on the seeded inputs of each test - the second way the oracle is
+pinned (the first is tests/test_oracle_golden.py).  What the reference computed on these inputs is stored in
+tests/golden/oracle_vs_reference.npz and tests/golden/qmix_action_mask.npz (tests/golden/make_golden.py writes both from the
+reference): small results whole, buffer contents as sha256 digests, initial weights as digests (the oracle rebuilds them
+from the same torch seed), final weights as a fixed element sample plus sum / abs-sum digests."""
+import os
 import random
-from argparse import Namespace
 
 import numpy as np
 import pytest
 import torch
-import torch.nn as nn
 
-from helpers import synth_rollout, fill_buffers, qmix_episode_stream, same_structure as _same
+from helpers import (synth_rollout, fill_buffers, qmix_episode_stream, array_digest, structure_digest, assert_same_init,
+                     assert_state_close)
 
-pytestmark = pytest.mark.reference
+G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+QMIX_BUFFER_KEYS = ('obs', 'actions', 'rewards', 'terminals', 'agent_mask')
 
 
 @pytest.fixture(scope="module")
 def ref():
-    from oracle.ref_loader import import_reference
-    return import_reference()
+    return np.load(os.path.join(G, "oracle_vs_reference.npz"), allow_pickle=False)
 
 
 @pytest.mark.parametrize("seed,use_gae", [(0, True), (1, True), (2, False)])
 def test_onpolicy_buffer_live(ref, seed, use_gae):
-    from gymnasium.spaces import Box, Discrete
-    from xuance.common.memory_tools import DummyOnPolicyBuffer
     from oracle.onpolicy import OnPolicyBufferOracle
     rng = np.random.default_rng(seed)
     N, T = 5, 33
     ro = synth_rollout(rng, N, T, (3,), obs_dtype=np.float32, p_term=0.1)
-    r = DummyOnPolicyBuffer(Box(-1, 1, (3,)), Discrete(4), {'old_logp': ()}, N, T, use_gae=use_gae)
     o = OnPolicyBufferOracle((3,), (), {'old_logp': ()}, N, T, use_gae=use_gae)
-    fill_buffers([r, o], ro, [(4, 1, np.float32(0.2)), (9, 3, 0.0), (20, 1, np.float32(-0.7))])
-    assert np.array_equal(r.returns, o.returns) and np.array_equal(r.advantages, o.advantages)
+    fill_buffers([o], ro, [(4, 1, np.float32(0.2)), (9, 3, 0.0), (20, 1, np.float32(-0.7))])
+    p = "onpolicy/%d" % seed
+    assert np.array_equal(ref[p + "/returns"], o.returns) and np.array_equal(ref[p + "/advantages"], o.advantages)
     idx = rng.permutation(N * T)[:50]
-    s1, s2 = r.sample(idx), o.sample(idx)
+    s2 = o.sample(idx)
     for k in ('obs', 'actions', 'returns', 'values', 'advantages'):
-        assert np.array_equal(s1[k], s2[k]) and s1[k].dtype == s2[k].dtype, k
+        s1k = ref[p + "/sample/" + k]
+        assert np.array_equal(s1k, s2[k]) and s1k.dtype == s2[k].dtype, k
 
 
 @pytest.mark.parametrize("alpha", [0.5, 0.6])
 def test_per_buffer_live(ref, alpha):
-    from gymnasium.spaces import Box, Discrete
-    from xuance.common.memory_tools import PerOffPolicyBuffer
+    """The reference ran with its float64 ``_max_priority`` replaced by a float32 one (canonical float32 rule,
+    oracle/replay.py docstring); its sum / min trees are kept as digests of their float64 leaf arrays."""
     from oracle.replay import PerReplayOracle
     rng = np.random.default_rng(int(alpha * 10))
     N, S, B = 4, 64, 32
-    r = PerOffPolicyBuffer(Box(-1, 1, (3,)), Discrete(4), None, N, N * S, B, alpha=alpha)
-    r._max_priority = np.ones(N, np.float32)       # canonical float32 rule (oracle/replay.py docstring)
     o = PerReplayOracle((3,), (), N, N * S, B, alpha=alpha)
+    g = {k: ref["per/%s/%s" % (alpha, k)] for k in ("step_choices", "weights", "sum_tree", "min_tree", "max_priority")}
+    j = 0
     for t in range(100):
         st = (rng.normal(size=(N, 3)).astype(np.float32), rng.integers(0, 4, N), rng.normal(size=N).astype(np.float32),
               rng.random(N) < 0.1, rng.normal(size=(N, 3)).astype(np.float32))
-        r.store(*st), o.store(*st)
+        o.store(*st)
         if t > 10 and t % 3 == 0:
             random.seed(t)
-            s1 = r.sample(0.4)
-            random.seed(t)
             s2 = o.sample(0.4)
-            assert np.array_equal(s1['step_choices'], s2['step_choices']) and np.array_equal(s1['weights'], s2['weights'])
+            assert np.array_equal(g["step_choices"][j], s2['step_choices']) and np.array_equal(g["weights"][j], s2['weights'])
             td = np.abs(rng.normal(size=B)).astype(np.float32)
             td[3] = 0
-            r.update_priorities(s1['step_choices'], td), o.update_priorities(s2['step_choices'], td)
-            for i in range(N):
-                assert np.array_equal(np.array(r._it_sum[i]._value, dtype=np.float64), o.sum[i].v.astype(np.float64))
-                assert np.array_equal(np.array(r._it_min[i]._value, dtype=np.float64), o.min[i].v.astype(np.float64))
-            assert np.array_equal(r._max_priority, o.max_priority)
+            o.update_priorities(s2['step_choices'], td)
+            assert g["sum_tree"][j] == array_digest(np.array([o.sum[i].v.astype(np.float64) for i in range(N)]))
+            assert g["min_tree"][j] == array_digest(np.array([o.min[i].v.astype(np.float64) for i in range(N)]))
+            assert np.array_equal(g["max_priority"][j], o.max_priority)
+            j += 1
+    assert j == len(g["step_choices"])
 
 
-def _qmix_pair(n, obs_dim, A, S, T, lr_decay=0.5):
-    from gymnasium.spaces import Discrete
-    from xuance.common import BaseCallback, AgentGrouping
-    from xuance.torch.rl_models.representations.rnn import Basic_RNN
-    from xuance.torch.rl_models.representations.agent_feature import AgentFeatureEncoder
-    from xuance.torch.rl_models.modules.identity_encoder import build_identity_encoder, IdentityFeatureFusion
-    from xuance.torch.rl_models.critics.base_critics import DiscreteActionValueCritic
-    from xuance.torch.rl_models.heads.q_mix_head import QMIX_Mixer
-    from xuance.torch.rl_models.architectures.multi_agent.value_factorization import MixingQNetwork
-    from xuance.torch.learners.multi_agent_rl.qmix_learner import QMIX_Learner
+def _qmix_oracle(n, obs_dim, A, S, total_iters, lr_decay=0.5):
+    """The oracle pair of the reference's QMIX model (use_rnn, shared GRU agent, mixer 32/32) + learner; built right after
+    torch.manual_seed it has the reference's initial weights (checked against the stored digests)."""
     from oracle.qmix import QMIXModelOracle, QMIXLearnerOracle
     keys = [f"agent_{i}" for i in range(n)]
-    rep = Basic_RNN(input_shape=(obs_dim,), hidden_sizes=None, initialize=nn.init.orthogonal_, activation=nn.ReLU,
-                    device='cpu', fc_hidden_sizes=[64], recurrent_hidden_size=64, N_recurrent_layers=1, dropout=0, rnn='GRU')
-    enc = AgentFeatureEncoder(rep, build_identity_encoder(n, 'none', None, 'cpu'), IdentityFeatureFusion(64, 0, 'concat'))
-    q = nn.ModuleDict({'shared': DiscreteActionValueCritic(enc, Discrete(A), [64], None, nn.init.orthogonal_, nn.ReLU, 'cpu')})
-    grouping = AgentGrouping.shared(keys)
-    model = MixingQNetwork(grouping, q, QMIX_Mixer(S, 32, 32, n, 'cpu'), use_rnn=True, device='cpu')
-    cfg = Namespace(distributed_training=False, episode_length=T, use_grad_clip=False, grad_clip_norm=10, device='cpu',
-                    model_dir='/tmp/x', running_steps=100000, parallels=4, use_parameter_sharing=True, use_rnn=True,
-                    use_actions_mask=False, learning_rate=7e-4, sync_frequency=2, double_q=True, n_epochs=1,
-                    start_training=0, gamma=0.99, end_factor_lr_decay=lr_decay)
-    lrn = QMIX_Learner(cfg, grouping, model, BaseCallback())
     om = QMIXModelOracle(n, obs_dim, A, S)
-    om.load_state_dict(model.state_dict(), strict=True)
     orc = QMIXLearnerOracle(om, keys, learning_rate=7e-4, sync_frequency=2, double_q=True, end_factor_lr_decay=lr_decay,
-                            total_iters=lrn.total_iters, detach_q_eval=True)   # the reference as it is (see oracle/qmix.py)
-    return keys, model, lrn, om, orc
+                            total_iters=total_iters, detach_q_eval=True)   # the reference as it is (see oracle/qmix.py)
+    return keys, om, orc
+
+
+def _fill_qmix_replay(ob, seed, keys, n_envs, T, obs_dim, A, S):
+    for ev in qmix_episode_stream(np.random.default_rng(seed), keys, n_envs, T, obs_dim, A, S, 5):
+        if ev[0] == 'store':
+            ob.store(**ev[1])
+        else:
+            ob.finish_path(ev[1], **ev[2])
+
+
+def _assert_qmix_replay(ob, keys, g, prefix):
+    got = [array_digest(ob.data[k][a]) for k in QMIX_BUFFER_KEYS for a in keys]
+    got += [array_digest(ob.data['filled']), array_digest(ob.data['state'])]
+    names = ["%s/%s" % (k, a) for k in QMIX_BUFFER_KEYS for a in keys] + ["filled", "state"]
+    for name, x, y in zip(names, g[prefix + "/digests"], got):
+        assert x == y, name
+    assert [ob.ptr, ob.size] == list(g[prefix + "/ptr_size"])
 
 
 def test_qmix_buffer_and_learner_live(ref):
-    from gymnasium.spaces import Box, Discrete
-    from xuance.common.memory_tools_marl import MARL_OffPolicyBuffer_RNN
     from oracle.qmix import EpisodeReplayOracle
     torch.manual_seed(0)
     n, obs_dim, A, S, T = 5, 72, 12, 98, 12
-    keys, model, lrn, om, orc = _qmix_pair(n, obs_dim, A, S, T)
-    init = {k: v.clone() for k, v in model.state_dict().items()}
+    keys, om, orc = _qmix_oracle(n, obs_dim, A, S, int(ref["qmix/total_iters"]))
+    assert_same_init(om.state_dict(), ref, "qmix/init")
+    init = {k: v.clone() for k, v in om.state_dict().items()}
     n_envs, C, Be = 3, 12, 6
-    rb = MARL_OffPolicyBuffer_RNN(agent_keys=keys, state_space=Box(-1, 1, (S,)),
-                                  obs_space={k: Box(-1, 1, (obs_dim,)) for k in keys},
-                                  act_space={k: Discrete(A) for k in keys}, n_envs=n_envs, buffer_size=C,
-                                  batch_size=Be, max_episode_steps=T, use_actions_mask=False)
     ob = EpisodeReplayOracle(keys, obs_dim, S, n_envs, C, Be, T)
-    for ev in qmix_episode_stream(np.random.default_rng(0), keys, n_envs, T, obs_dim, A, S, 5):
-        if ev[0] == 'store':
-            rb.store(**ev[1]), ob.store(**ev[1])
-        else:
-            rb.finish_path(ev[1], **ev[2]), ob.finish_path(ev[1], **ev[2])
-    for k in ('obs', 'actions', 'rewards', 'terminals', 'agent_mask'):
-        for a in keys:
-            assert np.array_equal(rb.data[k][a], ob.data[k][a]), k
-    assert np.array_equal(rb.data['filled'], ob.data['filled']) and np.array_equal(rb.data['state'], ob.data['state'])
-    assert rb.ptr == ob.ptr and rb.size == ob.size
+    _fill_qmix_replay(ob, 0, keys, n_envs, T, obs_dim, A, S)
+    _assert_qmix_replay(ob, keys, ref, "qmix/buffer")
     for it in range(3):
         np.random.seed(it)
-        s1 = rb.sample()
-        np.random.seed(it)
-        s2 = ob.sample()
-        i1, i2 = lrn.update(s1), orc.update(s2)
-        np.testing.assert_allclose(i1['loss_Q'], i2['loss_Q'], rtol=1e-5)
-        np.testing.assert_allclose(i1['predictQ'], i2['predictQ'], rtol=1e-5, atol=1e-7)
-        assert i1['learning_rate'] == i2['learning_rate']
-    sd1, sd2 = model.state_dict(), om.state_dict()
-    for k in sd1:
-        np.testing.assert_allclose(sd2[k].numpy(), sd1[k].numpy(), rtol=1e-5, atol=1e-6, err_msg=k)
+        i2 = orc.update(ob.sample())
+        i1 = ref["qmix/infos"][it]
+        np.testing.assert_allclose(i1[0], i2['loss_Q'], rtol=1e-5)
+        np.testing.assert_allclose(i1[1], i2['predictQ'], rtol=1e-5, atol=1e-7)
+        assert i1[2] == i2['learning_rate']
+    sd2 = om.state_dict()
+    assert_state_close(sd2, ref, "qmix/final", rtol=1e-5, atol=1e-6)
     # reference quirk pinned here: with use_rnn=True its agent networks never receive a gradient (only the mixer moves)
-    moved = {k for k in sd1 if k.startswith("individual_q_networks") and not torch.equal(sd1[k], init[k])}
+    assert len(ref["qmix/moved_agent_tensors"]) == 0, ref["qmix/moved_agent_tensors"]
+    moved = {k for k in sd2 if k.startswith("individual_q_networks") and not torch.equal(sd2[k], init[k])}
     assert not moved, moved
 
 
 def test_sac_learner_live(ref):
-    from copy import deepcopy
-    from gymnasium.spaces import Box
-    from xuance.common import BaseCallback
-    from xuance.torch.rl_models.representations.mlp import Basic_Identical
-    from xuance.torch.rl_models.actors.gaussian_actors import SAC_GaussianActor
-    from xuance.torch.rl_models.critics.twin_critics import TwinActionValueCritic
-    from xuance.torch.rl_models.architectures.single_agent.actor_critic import SoftActorCritic
-    from xuance.torch.learners import SAC_Learner
+    """The reference's SAC learner (MLP 256-256, automatic entropy tuning) built after torch.manual_seed(0)."""
     from oracle.sac import SACModelOracle, SACLearnerOracle
     torch.manual_seed(0)
     obs_dim, act_dim, B = 17, 6, 64
-    aspace = Box(-1, 1, (act_dim,), np.float32)
-    rep = Basic_Identical((obs_dim,), device='cpu')
-    actor = SAC_GaussianActor(rep, [256, 256], aspace, None, None, nn.LeakyReLU, nn.Tanh, 'cpu')
-    critic = TwinActionValueCritic(deepcopy(rep), aspace, [256, 256], None, None, nn.LeakyReLU, 'cpu')
-    model = SoftActorCritic(actor, critic)
-    cfg = Namespace(distributed_training=False, episode_length=1000, use_grad_clip=False, grad_clip_norm=0.5, device='cpu',
-                    model_dir='/tmp/x', running_steps=100000, parallels=4, start_training=0, training_frequency=1,
-                    learning_rate_actor=1e-3, learning_rate_critic=1e-3, tau=0.005, gamma=0.99, alpha=0.2,
-                    use_automatic_entropy_tuning=True, end_factor_lr_decay=0.7)
-    lrn = SAC_Learner(cfg, model, BaseCallback())
     om = SACModelOracle(obs_dim, act_dim)
-    om.load_state_dict(model.state_dict(), strict=True)
-    orc = SACLearnerOracle(om, end_factor_lr_decay=0.7, total_iters=lrn.total_iters)
+    assert_same_init(om.state_dict(), ref, "sac/init")
+    orc = SACLearnerOracle(om, end_factor_lr_decay=0.7, total_iters=int(ref["sac/total_iters"]))
     rng = np.random.default_rng(1)
     for it in range(3):
         s = {"obs": rng.normal(size=(B, obs_dim)).astype(np.float32),
@@ -172,55 +139,32 @@ def test_sac_learner_live(ref):
         torch.manual_seed(100 + it)
         n1 = torch.randn(B, act_dim)
         n2 = torch.randn(B, act_dim)
-        torch.manual_seed(100 + it)
-        i1 = lrn.update(**s)
         i2 = orc.update(n1, n2, **s)
-        for k in ("Qloss", "Ploss", "Qvalue", "alpha", "alpha_loss"):
-            np.testing.assert_allclose(i2[k], i1[k], rtol=1e-5, atol=1e-6, err_msg=k)
-    sd1, sd2 = model.state_dict(), om.state_dict()
-    for k in sd1:
-        np.testing.assert_allclose(sd2[k].numpy(), sd1[k].numpy(), rtol=1e-5, atol=1e-6, err_msg=k)
+        for k, v in zip(("Qloss", "Ploss", "Qvalue", "alpha", "alpha_loss"), ref["sac/infos"][it]):
+            np.testing.assert_allclose(i2[k], v, rtol=1e-5, atol=1e-6, err_msg=k)
+    assert_state_close(om.state_dict(), ref, "sac/final", rtol=1e-5, atol=1e-6)
 
 
 @pytest.mark.parametrize("kind", ["a2c", "pg", "ddqn"])
 def test_sibling_learners_live(ref, kind):
-    """A2C / PG / DDQN (SURVEY.md section 8f-3): oracle variants next to the reference learners."""
-    from gymnasium.spaces import Discrete
-    from xuance.common import BaseCallback
-    from xuance.torch.learners import A2C_Learner, PG_Learner, DDQN_Learner
-    from xuance.torch.rl_models.representations import AC_CNN_Atari, Basic_CNN
-    from xuance.torch.rl_models.heads import CategoricalActorHead, ValueHead
-    from xuance.torch.rl_models.architectures.single_agent.actor_critic import SharedActorCritic
-    from xuance.torch.rl_models.architectures.single_agent.deep_q_network import DeepQNetwork
+    """A2C / PG / DDQN (SURVEY.md section 8f-3): oracle variants next to the reference learners (NatureCNN at 84x84x4,
+    running_steps 40960, 32 envs, lr 2.5e-4 decaying to half, gradient clip 0.5, sync every 2 updates)."""
     from oracle.nets import SharedActorCriticOracle, DeepQNetworkOracle
     from oracle.learners import PPOLearnerOracle, DQNLearnerOracle
     torch.manual_seed(5)
     A, B = 5, 12
-    cfg = Namespace(distributed_training=False, episode_length=1000, use_grad_clip=True, grad_clip_norm=0.5, device="cpu",
-                    model_dir="/tmp/x", running_steps=4096 * 10, parallels=32, learning_rate=2.5e-4, end_factor_lr_decay=0.5,
-                    horizon_size=128, n_epochs=4, n_minibatch=4, vf_coef=0.25, ent_coef=0.01, gamma=0.99, sync_frequency=2,
-                    start_training=0, training_frequency=1)
+    p = "sibling/" + kind
+    total_iters = int(ref[p + "/total_iters"])
     rng = np.random.default_rng(3)
     if kind == "ddqn":
-        rep = Basic_CNN(input_shape=(84, 84, 4), kernels=[8, 4, 3], strides=[4, 2, 1], filters=[32, 64, 64],
-                        activation=nn.ReLU, device="cpu")
-        model = DeepQNetwork(rep, [512], Discrete(A), None, None, nn.ReLU, "cpu")
-        lrn = DDQN_Learner(cfg, model, BaseCallback())
         om = DeepQNetworkOracle(A)
-        om.load_state_dict(model.state_dict())
         orc = DQNLearnerOracle(om, learning_rate=2.5e-4, sync_frequency=2, use_grad_clip=True, end_factor_lr_decay=0.5,
-                               total_iters=lrn.total_iters, double_q=True)
+                               total_iters=total_iters, double_q=True)
     else:
-        rep = AC_CNN_Atari(input_shape=(84, 84, 4), kernels=[8, 4, 3], strides=[4, 2, 1], filters=[32, 64, 64],
-                           activation=nn.ReLU, device="cpu", fc_hidden_sizes=[512])
-        model = SharedActorCritic(rep, CategoricalActorHead(512, [], A, None, nn.init.orthogonal_, nn.ReLU, "cpu"),
-                                  ValueHead(512, [], None, nn.init.orthogonal_, nn.ReLU, "cpu"))
-        lrn = (A2C_Learner if kind == "a2c" else PG_Learner)(cfg, model, BaseCallback())
         om = SharedActorCriticOracle(A)
-        om.load_state_dict(model.state_dict())
         # a2c_learner.py:21: LinearLR(total_iters=config.running_steps); pg_learner.py:22: total_iters=self.total_iters
-        orc = PPOLearnerOracle(om, end_factor_lr_decay=0.5, kind=kind,
-                               total_iters=cfg.running_steps if kind == "a2c" else lrn.total_iters)
+        orc = PPOLearnerOracle(om, end_factor_lr_decay=0.5, kind=kind, total_iters=4096 * 10 if kind == "a2c" else total_iters)
+    assert_same_init(om.state_dict(), ref, p + "/init")
     for it in range(3):
         s = {"obs": rng.integers(0, 256, size=(B, 84, 84, 4), dtype=np.uint8).astype(np.float32),
              "actions": rng.integers(0, A, size=B).astype(np.float32),
@@ -228,114 +172,89 @@ def test_sibling_learners_live(ref, kind):
              "aux_batch": {"old_logp": np.zeros(B, np.float32)},
              "obs_next": rng.integers(0, 256, size=(B, 84, 84, 4), dtype=np.uint8).astype(np.float32),
              "rewards": rng.normal(size=B).astype(np.float32), "terminals": (rng.random(B) < 0.2).astype(np.float32)}
-        i1, i2 = lrn.update(**s), orc.update(**s)
+        i1, i2 = ref[p + "/infos"][it], orc.update(**s)
         if kind == "ddqn":
-            np.testing.assert_allclose(i2["Qloss"], i1["Qloss"], rtol=1e-5)
+            np.testing.assert_allclose(i2["Qloss"], i1[0], rtol=1e-5)
         else:
-            np.testing.assert_allclose(i2["actor_loss"], i1["actor-loss"], rtol=1e-5, atol=1e-7)
-            np.testing.assert_allclose(i2["entropy"], i1["entropy"], rtol=1e-5)
-    sd1, sd2 = model.state_dict(), om.state_dict()
-    for k in sd1:
-        np.testing.assert_allclose(sd2[k].numpy(), sd1[k].numpy(), rtol=1e-5, atol=1e-6, err_msg=k)
+            np.testing.assert_allclose(i2["actor_loss"], i1[0], rtol=1e-5, atol=1e-7)
+            np.testing.assert_allclose(i2["entropy"], i1[1], rtol=1e-5)
+    assert_state_close(om.state_dict(), ref, p + "/final", rtol=1e-5, atol=1e-6)
 
 
 def test_multi_agent_vector_env_live(ref):
     """DummyVecMultiAgentEnv + XuanCeMultiAgentEnvWrapper (the QMIX caller side, vector_envs/dummy/dummy_vec_maenv.py:17-84,
     environment/utils/wrapper.py:141-226) next to the live reference classes over the SAME raw synthetic environments:
     identical observations, reward / terminated dicts, truncation flags and infos (episode_step, episode_score, agent_mask,
-    avail_actions, state, reset_obs / reset_avail_actions / reset_state at episode ends) step for step."""
-    from xuance.environment.utils.wrapper import XuanCeMultiAgentEnvWrapper as RefWrapper
-    from xuance.environment.vector_envs.dummy.dummy_vec_maenv import DummyVecMultiAgentEnv as RefVec
+    avail_actions, state, reset_obs / reset_avail_actions / reset_state at episode ends) step for step.  The reference's
+    results are stored as helpers.structure_digest of each, equal exactly when helpers.same_structure would hold."""
     from xuance_b200.environment.ma_envs import SyntheticSMACEnv, XuanCeMultiAgentEnvWrapper
     from xuance_b200.environment.vector_envs.dummy_vec_maenv import DummyVecMultiAgentEnv
     kw = dict(n_agents=3, obs_dim=16, state_dim=20, n_actions=5, episode_limit=7, p_death=0.1)
     n_envs = 3
-    mk_ref = [lambda env_seed=0: RefWrapper(SyntheticSMACEnv(seed=env_seed, **kw)) for _ in range(n_envs)]
     mk_own = [lambda env_seed=0: XuanCeMultiAgentEnvWrapper(SyntheticSMACEnv(seed=env_seed, **kw)) for _ in range(n_envs)]
-    rv, ov = RefVec(mk_ref, 11), DummyVecMultiAgentEnv(mk_own, 11)
-    assert rv.num_envs == ov.num_envs and rv.agents == ov.agents and rv.num_agents == ov.num_agents
-    assert rv.max_episode_steps == ov.max_episode_steps and rv.state_space.shape == ov.state_space.shape
-    (ro, ri), (oo, oi) = rv.reset(), ov.reset()
-    _same(ro, oo, "reset obs"), _same(ri, oi, "reset info")
+    ov = DummyVecMultiAgentEnv(mk_own, 11)
+    assert list(ref["maenv/attrs"]) == [ov.num_envs, ov.num_agents, ov.max_episode_steps]
+    assert list(ref["maenv/agents"]) == list(ov.agents) and tuple(ref["maenv/state_shape"]) == ov.state_space.shape
+    names, digests = list(ref["maenv/names"]), ref["maenv/digests"]
+    oo, oi = ov.reset()
+    assert digests[0][0] == structure_digest(oo), "reset obs"
+    assert digests[0][1] == structure_digest(oi), "reset info"
     rng = np.random.default_rng(2)
     ends = 0
     for t in range(40):
-        # a random AVAILABLE action per agent (the same for both stacks)
-        acts = [{a: int(rng.choice(np.flatnonzero(rv.buf_avail_actions[e][a]))) for a in rv.agents} for e in range(n_envs)]
-        r, o = rv.step(acts), ov.step(acts)
-        for name, x, y in zip(("obs", "rewards", "terminated", "truncated", "infos"), r, o):
-            _same(x, y, "t=%d %s" % (t, name))
-        _same(rv.buf_state, ov.buf_state, "state"), _same(rv.buf_avail_actions, ov.buf_avail_actions, "avail")
-        ends += sum("reset_obs" in i for i in r[4])
-    assert ends >= 5                                    # episode ends (death of all agents / truncation) were exercised
-    rv.close(), ov.close()
+        # a random AVAILABLE action per agent (the reference drew from the same availability, checked step by step)
+        acts = [{a: int(rng.choice(np.flatnonzero(ov.buf_avail_actions[e][a]))) for a in ov.agents} for e in range(n_envs)]
+        o = ov.step(acts)
+        for name, x, y in zip(names, digests[t + 1], tuple(o) + (ov.buf_state, ov.buf_avail_actions)):
+            assert x == structure_digest(y), "t=%d %s" % (t, name)
+        ends += sum("reset_obs" in i for i in o[4])
+    assert ends == int(ref["maenv/episode_ends"]) and ends >= 5   # episode ends (death of all agents / truncation) exercised
+    ov.close()
 
 
-def test_qmix_action_mask_variant_against_the_reference_with_its_slice_corrected(ref, monkeypatch):
+def test_qmix_action_mask_variant_against_the_reference_with_its_slice_corrected():
     """use_rnn=True with use_actions_mask=True: the reference slices the AGENT axis of the availability mask
     (iql_learner.py:78, ``[:, 1:]``) and raises; the evidently intended statement slices the time axis (``[:, :, 1:]``).
     The oracle's masked variant (and through it xb_qmix_select_fwd's masked arg-max / target, tests/test_gpu_qmix.py) is pinned
-    here against the LIVE reference learner with that ONE expression corrected at run time - the reference source is read
-    from /root/reference, patched in memory and executed; nothing of it is stored in this repository."""
-    import inspect
-    import textwrap
-    from gymnasium.spaces import Box, Discrete
-    from xuance.common.memory_tools_marl import MARL_OffPolicyBuffer_RNN
-    from xuance.torch.learners.multi_agent_rl import iql_learner as iql
+    here against the reference learner with that ONE expression corrected in memory (tests/golden/qmix_action_mask.npz;
+    nothing of the reference's source is stored in this repository).  The reference buffer's availability masks are stored
+    whole; the oracle buffer rebuilds its other contents from the same seeded stream."""
+    from oracle.qmix import EpisodeReplayOracle
+    g = np.load(os.path.join(G, "qmix_action_mask.npz"), allow_pickle=False)
     torch.manual_seed(1)
     n, obs_dim, A, S, T = 4, 24, 7, 30, 9
-    keys, model, lrn, om, orc = _qmix_pair(n, obs_dim, A, S, T)
-    lrn.use_actions_mask = lrn.config.use_actions_mask = True
+    keys, om, orc = _qmix_oracle(n, obs_dim, A, S, int(g["total_iters"]))
+    assert_same_init(om.state_dict(), g, "init")
     orc.use_actions_mask = True
     n_envs, C, Be = 3, 12, 6
-    rb = MARL_OffPolicyBuffer_RNN(agent_keys=keys, state_space=Box(-1, 1, (S,)),
-                                  obs_space={k: Box(-1, 1, (obs_dim,)) for k in keys},
-                                  act_space={k: Discrete(A) for k in keys}, n_envs=n_envs, buffer_size=C,
-                                  batch_size=Be, max_episode_steps=T, use_actions_mask=True,
-                                  avail_actions_shape={k: (A,) for k in keys})
-    rng = np.random.default_rng(4)
+    ob = EpisodeReplayOracle(keys, obs_dim, S, n_envs, C, Be, T)
+    _fill_qmix_replay(ob, 3, keys, n_envs, T, obs_dim, A, S)
+    _assert_qmix_replay(ob, keys, g, "buffer")
+    avail = g["buffer/avail_actions"]                       # [n_agents, buffer_size, T + 1, A]
+    assert avail.shape == (n, C, T + 1, A)
 
-    def avail(shape_prefix):
-        a = rng.random(shape_prefix + (A,)) < 0.6
-        a[..., 0] = True                                    # never an all-unavailable row
-        return a
-    for ev in qmix_episode_stream(np.random.default_rng(3), keys, n_envs, T, obs_dim, A, S, 5):
-        if ev[0] == 'store':
-            rb.store(avail_actions={k: avail((n_envs,)) for k in keys}, **ev[1])
-        else:
-            rb.finish_path(ev[1], avail_actions={k: avail(()) for k in keys}, **ev[2])
-    np.random.seed(0)
-    sample = rb.sample()
-    assert sample['avail_actions'][keys[0]].shape == (Be, T + 1, A)
+    def sample(seed):                                       # MARL_OffPolicyBuffer_RNN.sample: np.random.choice(size, batch)
+        np.random.seed(seed)
+        episodes = np.random.choice(ob.size, Be)
+        s = ob.gather(episodes)
+        s['avail_actions'] = {a: avail[i][episodes] for i, a in enumerate(keys)}
+        return s
+    assert tuple(g["sample_avail_shape"]) == sample(0)['avail_actions'][keys[0]].shape == (Be, T + 1, A)
     # 1. the reference as it is cannot run this configuration
-    snap = {k: v.clone() for k, v in model.state_dict().items()}
-    with pytest.raises((RuntimeError, IndexError)):
-        lrn.update(sample)
-    model.load_state_dict(snap)
-    lrn.iterations = 0
+    assert str(g["unpatched_error"]) in ("RuntimeError", "IndexError")
+    assert int(g["bad_slice_count"]) == 1
     # 2. the same learner with the one slice corrected
-    src = textwrap.dedent(inspect.getsource(iql.IQL_Learner._forward_transitions))
-    bad = "batch.avail_actions.group(group)[:, 1:]"
-    assert src.count(bad) == 1, "the reference's masked RNN branch changed - re-read iql_learner.py:60-81"
-    scope = {}
-    exec(compile(src.replace(bad, "batch.avail_actions.group(group)[:, :, 1:]"), "iql_learner.py (slice corrected)", "exec"),
-         vars(iql), scope)
-    monkeypatch.setattr(iql.IQL_Learner, "_forward_transitions", scope["_forward_transitions"])
+    snap = {k: v.clone() for k, v in om.state_dict().items()}
     for it in range(3):
-        np.random.seed(10 + it)
-        s = rb.sample()
-        i1, i2 = lrn.update(s), orc.update(s)
-        np.testing.assert_allclose(i1['loss_Q'], i2['loss_Q'], rtol=1e-5)
-        np.testing.assert_allclose(i1['predictQ'], i2['predictQ'], rtol=1e-5, atol=1e-7)
-    sd1, sd2 = model.state_dict(), om.state_dict()
-    for k in sd1:
-        np.testing.assert_allclose(sd2[k].numpy(), sd1[k].numpy(), rtol=1e-5, atol=1e-6, err_msg=k)
+        i1, i2 = g["infos"][it], orc.update(sample(10 + it))
+        np.testing.assert_allclose(i1[0], i2['loss_Q'], rtol=1e-5)
+        np.testing.assert_allclose(i1[1], i2['predictQ'], rtol=1e-5, atol=1e-7)
+    assert_state_close(om.state_dict(), g, "final", rtol=1e-5, atol=1e-6)
     # the masks mattered: the same first update without them has a different loss
-    _, _, _, om_m, orc_m = _qmix_pair(n, obs_dim, A, S, T)
-    _, _, _, om_u, orc_u = _qmix_pair(n, obs_dim, A, S, T)
+    _, om_m, orc_m = _qmix_oracle(n, obs_dim, A, S, int(g["total_iters"]))
+    _, om_u, orc_u = _qmix_oracle(n, obs_dim, A, S, int(g["total_iters"]))
     om_m.load_state_dict(snap, strict=True), om_u.load_state_dict(snap, strict=True)
     om_m.copy_target(), om_u.copy_target()
     orc_m.use_actions_mask = True
-    np.random.seed(10)
-    s = rb.sample()
+    s = sample(10)
     assert abs(orc_m.update(s)['loss_Q'] - orc_u.update(s)['loss_Q']) > 1e-6
