@@ -103,6 +103,23 @@ int xb_ppo_loss_fwd_bwd(const float *logits, const float *value, const float *ac
                         int64_t B, int A, int64_t B_total, float clip_range, float vf_coef, float ent_coef,
                         int loss_kind, float *dlogits, float *dvalue, float *stats, double *scratch, void *stream);
 
+/* ---------------------------------------------------------------- K4-G: Gaussian-policy PPO loss ------
+ * K4 for a diagonal Gaussian policy (GaussianActorHead + DiagGaussianDistribution, actor_head.py:45-72,
+ * distributions.py:165-197): torch.distributions.Normal(mu, exp(log_std)) with log-prob and entropy summed over D,
+ *   logp_b = sum_d [-(a-mu)^2/(2 sigma^2) - log sigma - log sqrt(2 pi)];  H = sum_d [1/2 + log sqrt(2 pi) + log sigma]
+ * and the same surrogate, value loss, loss_kind, B_total scaling and stats[8] layout as xb_ppo_loss_fwd_bwd.
+ * mu[B,D] is the head's output after activation_action, log_std[D] the head's parameter, actions[B,D] float32.
+ * Writes dmu[B,D], dvalue[B] and dlog_std[D] = sum_b dloss/dlogp_b * ((a-mu)^2/sigma^2 - 1) - ent_coef*B/B_total,
+ * a reduction over every row that is bit-identical from run to run (fixed-order double sums, no float atomics).
+ * scratch: the K4 scratch (xb_scratch_doubles()); col_scratch: xb_gaussian_scratch_doubles(D) doubles for the
+ * per-dimension block partials (need not be zeroed).  1 <= D <= 64 (XB_ERANGE above). */
+int64_t xb_gaussian_scratch_doubles(int D);
+int xb_ppo_gaussian_loss_fwd_bwd(const float *mu, const float *log_std, const float *value, const float *actions,
+                                 const float *old_logp, const float *adv, const float *ret, int64_t B, int D,
+                                 int64_t B_total, float clip_range, float vf_coef, float ent_coef, int loss_kind,
+                                 float *dmu, float *dvalue, float *dlog_std, float *stats, double *scratch,
+                                 double *col_scratch, void *stream);
+
 /* ---------------------------------------------------------------- K5: prioritized-replay trees -------
  * Replaces SumSegmentTree/MinSegmentTree (xuance/common/segtree_tool.py:4-220) and their use in
  * PerOffPolicyBuffer (memory_tools.py:505-598).  One (sum,min) pair PER ENV, float32 nodes, heap layout
@@ -218,6 +235,13 @@ int xb_soft_update(float *target, const float *source, int64_t n, float tau, voi
  *   else                   : a_n = first argmax_i p_i               (deterministic_sample)
  *   outputs (each nullable, at least one): actions_f32[N] (the float32 the buffers store), actions_i32[N] (for the
  *   host-side env step), logp[N] = log_softmax(logits)[a], entropy[N] = -sum p log p.
+ * xb_gaussian_act: DiagGaussianDistribution over Normal(mu[N,D], exp(log_std[D])) (distributions.py:165-197), D <= 64.
+ *   forced_actions[N,D] != NULL : a = forced_actions                (log_prob / entropy of given actions)
+ *   else noise[N,D] != NULL     : a = mu + noise * sigma, rounded after the product and after the sum as Normal.rsample
+ *                                 (noise: standard normal draws supplied by the caller)
+ *   else                        : a = mu                            (deterministic_sample)
+ *   outputs (each nullable, at least one): actions_f32[N,D] (what the env steps with and the buffer stores),
+ *   logp[N] = sum_d Normal.log_prob(a), entropy[N] = sum_d Normal.entropy().
  * xb_rms_update_normalize: x[N,D] float32.
  *   update != 0: (mean, var)[D] <- parallel-variance merge with the batch moments, float32 in the reference's operation
  *                order; `count` is the running count BEFORE the merge (host state, Python float in the reference).
@@ -226,6 +250,8 @@ int xb_soft_update(float *target, const float *source, int64_t n, float tau, voi
  */
 int xb_categorical_act(const float *logits, const float *uniforms, const float *forced_actions, int N, int A,
                        float *actions_f32, int32_t *actions_i32, float *logp, float *entropy, void *stream);
+int xb_gaussian_act(const float *mu, const float *log_std, const float *noise, const float *forced_actions, int N, int D,
+                    float *actions_f32, float *logp, float *entropy, void *stream);
 int xb_rms_update_normalize(const float *x, int N, int64_t D, float *mean, float *var, double count, int update,
                             float *out, float clip_range, float eps, void *stream);
 

@@ -1,9 +1,10 @@
 #!/usr/bin/env python
 """Secondary measurements for BASELINE configs 3-5 (parity-test cases, not the headline): sample + update throughput of
 DQN+PER (2^20-transition HBM replay, B=512), SAC (1M replay, B=1024) and QMIX (5 agents x 72-d, T=60, 32 episodes)
-on one B200, next to the oracle port of the reference's torch-CPU path on the host.  Prints one JSON object.
+on one B200, next to the oracle port of the reference's torch-CPU path on the host.  Also continuous-action PPO
+(ppo_gaussian: configs/ppo/mujoco.yaml shapes, one GPU).  Prints one JSON object.
 
-    python tools/algo_bench.py [--iters 200] [--cpu-iters 5] [--no-cpu] [--graph]
+    python tools/algo_bench.py [--iters 200] [--cpu-iters 5] [--no-cpu] [--graph] [--only perdqn,sac,qmix,ppo_gaussian]
     torchrun --nnodes=1 --nproc-per-node G --master-addr 127.0.0.1 tools/algo_bench.py --no-cpu --graph    (G GPUs)
 
 Multi-GPU (BASELINE configs 3 and 5 are multi-GPU configurations): one process per GPU; the replay is sharded (envs / episodes
@@ -184,12 +185,67 @@ def bench_qmix(args, Be=32):
     return out
 
 
+def _card():
+    """Name and power limit of the card the numbers were measured on (read-only query)."""
+    import subprocess
+    try:
+        q = subprocess.run(["nvidia-smi", "-i", str(LOCAL), "--query-gpu=name,power.limit", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        q = ""
+    return {"gpu": torch.cuda.get_device_name(LOCAL), "nvidia_smi_name_power_limit": q}
+
+
+def bench_ppo_gaussian(args):
+    """PPO-Clip with a Gaussian policy (K4-G in every update): configs/ppo/mujoco.yaml - 17-d obs, 6-d action, Basic_Identical
+    + MLP 256-256, 16 epochs x 8 minibatches of a 16 x 256 rollout (B = 512) - and a large-batch row (256 x 256 rollout,
+    B = 8192).  train_epochs runs on a filled buffer (GAE included); env-steps/s = rollout steps consumed per second of
+    train_epochs.  The CPU arm is the oracle's update (torch on the host) at the same B."""
+    from xuance_b200.common import Box
+    from xuance_b200.common.common_tools import get_arguments
+    from xuance_b200.torch.agents import PPO_Agent
+    from oracle.gaussian import GaussianActorCriticOracle, PPOGaussianLearnerOracle
+    od, ad = 17, 6
+    out = {"card": _card()}
+    for name, parallels in (("mujoco_B512", 16), ("large_B8192", 256)):
+        cfg = get_arguments("ppo", "mujoco", parser_args=Namespace(device=DEV, parallels=parallels, logger=None,
+                                                                    use_cuda_graph=args.graph, model_dir="/tmp/xb_bench"))
+        agent = PPO_Agent(cfg, None, Box(-np.inf, np.inf, (od,), np.float32), Box(-1, 1, (ad,), np.float32))
+        mem, N, T = agent.memory, agent.n_envs, agent.horizon_size
+        g = torch.Generator(device=DEV).manual_seed(0)
+        for t in range(T):
+            mem.store(torch.randn((N, od), device=DEV, generator=g), torch.rand((N, ad), device=DEV, generator=g) * 2 - 1,
+                      torch.randn(N, device=DEV, generator=g), torch.randn(N, device=DEV, generator=g),
+                      torch.zeros(N, device=DEV), {"old_logp": torch.randn(N, device=DEV, generator=g) - 5.0})
+        mem.finish_paths(np.zeros(N, np.float32))
+        B = agent.batch_size
+        n_upd = cfg.n_epochs * cfg.n_minibatch
+        reps = max(1, args.iters // n_upd)
+        dt = timed(lambda: agent.train_epochs(cfg.n_epochs), reps, warm=2)
+        row = {"config": "PPO Gaussian, %d envs x %d steps, %d epochs x %d minibatches, B=%d, MLP 256-256, cuda_graph=%s"
+                         % (N, T, cfg.n_epochs, cfg.n_minibatch, B, bool(args.graph)),
+               "gpu_updates_per_s": n_upd / dt, "gpu_ms_per_update": dt / n_upd * 1e3,
+               "gpu_train_epochs_s": dt, "gpu_env_steps_per_s": N * T / dt}
+        if not args.no_cpu:
+            torch.manual_seed(0)
+            ol = PPOGaussianLearnerOracle(GaussianActorCriticOracle(od, ad), learning_rate=4e-4, ent_coef=0.0)
+            rng = np.random.default_rng(0)
+            s = {"obs": rng.normal(size=(B, od)).astype(np.float32), "actions": rng.uniform(-1, 1, (B, ad)).astype(np.float32),
+                 "returns": rng.normal(size=B).astype(np.float32), "advantages": rng.normal(size=B).astype(np.float32),
+                 "aux_batch": {"old_logp": (rng.normal(size=B) - 5.0).astype(np.float32)}}
+            cdt = cpu_timed(lambda: ol.update(**s), max(args.cpu_iters, 20))
+            row.update(cpu_updates_per_s=1 / cdt, cpu_ms_per_update=cdt * 1e3, cpu_threads=torch.get_num_threads(),
+                       speedup=cdt / (dt / n_upd))
+        out[name] = row
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--iters", type=int, default=200)
     ap.add_argument("--cpu-iters", type=int, default=5)
     ap.add_argument("--no-cpu", action="store_true")
-    ap.add_argument("--only", default="")
+    ap.add_argument("--only", default="", help="comma-separated subset of perdqn,sac,qmix,ppo_gaussian")
     ap.add_argument("--graph", action="store_true", help="capture the learners' device update in a CUDA graph")
     ap.add_argument("--compute", default="fp32", choices=["fp32", "tc"], help="pixel encoder of the PER-DQN network")
     args = ap.parse_args()
@@ -211,6 +267,8 @@ def main():
     if not only or "qmix" in only:
         res["qmix"] = bench_qmix(args)
         res["qmix_4096"] = bench_qmix(Namespace(**{**vars(args), "iters": 20, "no_cpu": True}), Be=1024)
+    if (not only or "ppo_gaussian" in only) and WORLD == 1:
+        res["ppo_gaussian"] = bench_ppo_gaussian(args)
     res["cuda_graph"] = bool(args.graph)
     res["n_gpus"] = WORLD
     if RANK == 0:

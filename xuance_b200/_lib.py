@@ -30,6 +30,9 @@ _SIGNATURES = {
     "xb_adv_normalize": (c_int, [_P, c_int64, _P, _P]),
     "xb_ppo_loss_fwd_bwd": (c_int, [_P, _P, _P, _P, _P, _P, c_int64, c_int, c_int64, c_float, c_float, c_float,
                                     c_int, _P, _P, _P, _P, _P]),
+    "xb_gaussian_scratch_doubles": (c_int64, [c_int]),
+    "xb_ppo_gaussian_loss_fwd_bwd": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64, c_int, c_int64, c_float, c_float,
+                                             c_float, c_int, _P, _P, _P, _P, _P, _P, _P]),
     "xb_per_insert": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_float, _P]),
     "xb_per_sample": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, c_int64, c_float, _P, _P, _P, _P]),
     "xb_per_update": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, c_float, _P]),
@@ -58,6 +61,7 @@ _SIGNATURES = {
                                    _P, _P]),
     "xb_wgrad_reduce": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_float, _P, c_int, _P]),
     "xb_categorical_act": (c_int, [_P, _P, _P, c_int, c_int, _P, _P, _P, _P, _P]),
+    "xb_gaussian_act": (c_int, [_P, _P, _P, _P, c_int, c_int, _P, _P, _P, _P]),
     "xb_rms_update_normalize": (c_int, [_P, c_int, c_int64, _P, _P, c_double, c_int, _P, c_float, c_float, _P]),
     "xb_sac_actor_loss": (c_int, [_P, _P, _P, _P, c_int64, c_int64, _P, _P, _P, _P, _P, _P]),
     "xb_sac_critic_loss": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_float, c_int64, c_int64, _P, _P, _P, _P, _P, _P]),

@@ -315,16 +315,21 @@ class DummyOnPolicyBuffer(Buffer):
     # collected straight into the K1 staging block; after the env step only rewards / terminals cross PCIe.
     def policy_slots(self):
         """float32 [N] device views {'actions', 'values', 'aux:<key>'...} of the persistent staging block that
-        ``store_staged`` hands to K1.  Fill them (e.g. K10 ``xb_categorical_act``) before calling ``store_staged``."""
-        if not self._scalar_action:
-            raise NotImplementedError("policy_slots: scalar (Discrete) action spaces only")
+        ``store_staged`` hands to K1.  Fill them (e.g. K10 ``xb_categorical_act``) before calling ``store_staged``.
+        For a vector action space 'actions' is a float32 [N, *action_shape] staging tensor of its own (K10-G
+        ``xb_gaussian_act`` writes it), stored with the same rows path ``store`` uses for vector actions."""
         if getattr(self, "_dev_scal", None) is None:
             N = self.n_envs
             self._dev_scal = torch.zeros((self._n_store, N), dtype=torch.float32, device=self.device)
+            self._dev_act = None if self._scalar_action else \
+                torch.zeros((N,) + self._act_shape, dtype=torch.float32, device=self.device)
             self._stage_rt = [torch.zeros((2, N), dtype=torch.float32).pin_memory() for _ in range(2)]
             self._stage_rt_evt = [None, None]
             self._stage_rt_i = 0
-        return {n: self._dev_scal[self._fid[n]] for n in self._names[2:self._n_store]}
+        slots = {n: self._dev_scal[self._fid[n]] for n in self._names[2:self._n_store]}
+        if not self._scalar_action:
+            slots["actions"] = self._dev_act
+        return slots
 
     def store_staged(self, obs, rews, terminals):
         """``store`` for a step whose actions / values / aux already sit in ``policy_slots()``: ``obs`` is the CUDA
@@ -346,6 +351,8 @@ class DummyOnPolicyBuffer(Buffer):
         obs_d = obs.to(self.obs_dtype).reshape(N, -1).contiguous()
         _lib.call("xb_rollout_store", _lib.ptr(self._obs), _lib.ptr(obs_d), obs_d.shape[1] * obs_d.element_size(),
                   _lib.ptr(self._fields), _lib.ptr(self._dev_scal), self._n_store, N, T, t)
+        if not self._scalar_action:
+            self._store_rows(self._act_rows, self._dev_act, t)
         self.ptr = (self.ptr + 1) % self.n_size
         self.size = min(self.size + 1, self.n_size)
 

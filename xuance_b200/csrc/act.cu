@@ -97,6 +97,59 @@ extern "C" int xb_categorical_act(const float *logits, const float *uniforms, co
 }
 
 // =====================================================================================================
+// K10-G  xb_gaussian_act
+// =====================================================================================================
+// DiagGaussianDistribution over Normal(mu, exp(log_std)) (modules/distributions.py:165-197), one thread per row:
+//   a = mu + noise * sigma  (Normal.rsample: one product, one sum, each rounded - no fused multiply-add)
+//   logp = sum_d [-(a-mu)^2 / (2 var) - log sigma - log sqrt(2 pi)],  entropy = sum_d [0.5 + 0.5 log(2 pi) + log sigma]
+// The reference draws with Normal.sample from torch's RNG; as for K10 the draw is defined on the caller's noise.
+template <int D_MAX>
+__global__ void __launch_bounds__(128) gaussian_act_kernel(const float *__restrict__ mu,
+                                                           const float *__restrict__ log_std,
+                                                           const float *__restrict__ noise,
+                                                           const float *__restrict__ forced, int N, int D,
+                                                           float *__restrict__ act_f, float *__restrict__ logp,
+                                                           float *__restrict__ entropy) {
+    const int n = blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= N) return;
+    const int64_t o = (int64_t)n * D;
+    float lp = 0.f, ent = 0.f;
+#pragma unroll
+    for (int d = 0; d < D_MAX; ++d) {
+        if (d < D) {
+            const float sigma = expf(log_std[d]);
+            const float m = mu[o + d];
+            float a = m;
+            if (forced) a = forced[o + d];
+            else if (noise) a = __fadd_rn(m, __fmul_rn(noise[o + d], sigma));
+            const float diff = a - m, log_scale = logf(sigma);
+            lp += -(diff * diff) / (2.0f * (sigma * sigma)) - log_scale - (float)XB_LOG_SQRT_2PI;
+            ent += (float)(0.5 + XB_LOG_SQRT_2PI) + log_scale;
+            if (act_f) act_f[o + d] = a;
+        }
+    }
+    if (logp) logp[n] = lp;
+    if (entropy) entropy[n] = ent;
+}
+
+extern "C" int xb_gaussian_act(const float *mu, const float *log_std, const float *noise, const float *forced_actions,
+                               int N, int D, float *actions_f32, float *logp, float *entropy, void *stream) {
+    if (!mu || !log_std || N <= 0 || D <= 0) return XB_EINVAL;
+    if (!actions_f32 && !logp && !entropy) return XB_EINVAL;
+    if (D > 64) return XB_ERANGE;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int grid = (N + 127) / 128;
+#define XB_GACT(DM) \
+    gaussian_act_kernel<DM><<<grid, 128, 0, s>>>(mu, log_std, noise, forced_actions, N, D, actions_f32, logp, entropy)
+    if (D <= 8) XB_GACT(8);
+    else if (D <= 18) XB_GACT(18);
+    else if (D <= 32) XB_GACT(32);
+    else XB_GACT(64);
+#undef XB_GACT
+    return xb_launch_status();
+}
+
+// =====================================================================================================
 // K11  xb_rms_update_normalize
 // =====================================================================================================
 // RunningMeanStd.update + Agent._process_observation for a float32 batch x[N,D] (common/statistic_tools.py:117-185,

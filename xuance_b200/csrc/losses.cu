@@ -164,6 +164,180 @@ extern "C" int xb_ppo_loss_fwd_bwd(const float *logits, const float *value, cons
 }
 
 // =====================================================================================================
+// K4-G  xb_ppo_gaussian_loss_fwd_bwd
+// =====================================================================================================
+// The same losses for a diagonal Gaussian policy, torch.distributions.Normal(mu, exp(log_std)) as ppo_learner.py:46-60
+// uses it through DiagGaussianDistribution (log_prob and entropy summed over the action dimensions):
+//   logp_b = sum_d [-(a-mu)^2 / (2 var) - log sigma - log sqrt(2 pi)],  H = sum_d [0.5 + 0.5 log(2 pi) + log sigma]
+//   d logp_b / d mu_d = (a-mu)/var,  d logp_b / d log_std_d = (a-mu)^2/var - 1,  d H / d log_std_d = 1
+// dlog_std is a reduction over every row: per-thread float partials, then warp / block / grid sums in double and in a
+// fixed order (deterministic), the block partials in col_scratch[D][XB_MAX_PARTIALS] and the logged statistics in the
+// K4 scratch, both finished by the last block to arrive.
+extern "C" int64_t xb_gaussian_scratch_doubles(int D) {
+    return (D <= 0 || D > 64) ? 0 : (int64_t)D * XB_MAX_PARTIALS;
+}
+
+template <int D_MAX>
+__global__ void __launch_bounds__(256) ppo_gaussian_loss_kernel(
+    const float *__restrict__ mu, const float *__restrict__ log_std, const float *__restrict__ value,
+    const float *__restrict__ actions, const float *__restrict__ old_logp, const float *__restrict__ adv,
+    const float *__restrict__ ret, int64_t B, int D, int64_t B_total, float inv_bt, float clip, float vf_coef,
+    float ent_coef, int loss_kind, float *__restrict__ dmu, float *__restrict__ dvalue, float *__restrict__ dlog_std,
+    float *__restrict__ stats, double *__restrict__ scratch, double *__restrict__ col_scratch) {
+    __shared__ double red[6 * 32];
+    __shared__ double col_red[D_MAX * 8];  // [d][warp], 8 warps of 256 threads
+    __shared__ float s_inv_var[D_MAX], s_two_var[D_MAX], s_log_scale[D_MAX];
+    __shared__ float s_entropy;
+    __shared__ bool is_last;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    if (threadIdx.x < D) {
+        const float sigma = expf(log_std[threadIdx.x]);
+        const float var = sigma * sigma;  // Normal.log_prob: var = scale ** 2, log_scale = scale.log()
+        s_inv_var[threadIdx.x] = 1.0f / var;
+        s_two_var[threadIdx.x] = 2.0f * var;
+        s_log_scale[threadIdx.x] = logf(sigma);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float h = 0.f;
+        for (int d = 0; d < D; ++d) h += (float)(0.5 + XB_LOG_SQRT_2PI) + s_log_scale[d];
+        s_entropy = h;
+    }
+    __syncthreads();
+    const float lo = 1.0f - clip, hi = 1.0f + clip, ent = s_entropy;
+    double acc[6] = {0, 0, 0, 0, 0, 0};  // a_loss, c_loss, entropy, v, clipped count, (unused)
+    float col[D_MAX];                     // this thread's share of sum_b dlogp_b * ((a-mu)^2/var - 1)
+#pragma unroll
+    for (int d = 0; d < D_MAX; ++d) col[d] = 0.f;
+    for (int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; b < B; b += (int64_t)gridDim.x * blockDim.x) {
+        const float *mr = mu + b * D, *ar = actions + b * D;
+        float diff[D_MAX];
+        float logp = 0.f;
+#pragma unroll
+        for (int d = 0; d < D_MAX; ++d) {
+            if (d < D) {
+                diff[d] = ar[d] - mr[d];
+                logp += -(diff[d] * diff[d]) / s_two_var[d] - s_log_scale[d] - (float)XB_LOG_SQRT_2PI;
+            }
+        }
+        const float ad = adv[b];
+        float ratio = 1.f, smin, d_logp;
+        if (loss_kind == 0) {  // PPO-Clip surrogate (same arithmetic as K4)
+            ratio = expf(logp - old_logp[b]);
+            const float rc = fminf(fmaxf(ratio, lo), hi);
+            const float s1 = rc * ad, s2 = ad * ratio;
+            smin = fminf(s1, s2);
+            float g1 = s1 < s2 ? 1.f : (s1 == s2 ? 0.5f : 0.f);
+            float g2 = s2 < s1 ? 1.f : (s1 == s2 ? 0.5f : 0.f);
+            const bool inside = ratio >= lo && ratio <= hi;
+            d_logp = -inv_bt * ad * ((inside ? g1 : 0.f) + g2) * ratio;
+        } else {  // plain policy gradient: a_loss = -mean(w * logp)
+            smin = ad * logp;
+            d_logp = -inv_bt * ad;
+        }
+        float *gr = dmu + b * D;
+#pragma unroll
+        for (int d = 0; d < D_MAX; ++d) {
+            if (d < D) {
+                const float z = diff[d] * s_inv_var[d];
+                gr[d] = d_logp * z;
+                col[d] += d_logp * (z * diff[d] - 1.f);
+            }
+        }
+        const float v = value[b], dv = v - ret[b];
+        dvalue[b] = vf_coef * 2.f * dv * inv_bt;
+        acc[0] += (double)(-smin);
+        acc[1] += (double)dv * (double)dv;
+        acc[2] += (double)ent;
+        acc[3] += (double)v;
+        acc[4] += (ratio < lo || ratio > hi) ? 1.0 : 0.0;
+    }
+    // per-dimension block partial: warps in shuffle order, then the block's warps in index order
+#pragma unroll
+    for (int d = 0; d < D_MAX; ++d) {
+        if (d < D) {
+            const double s = warp_sum_d((double)col[d]);
+            if (lane == 0) col_red[d * 8 + warp] = s;
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < D) {
+        double s = 0.0;
+        for (int w = 0; w < nwarps; ++w) s += col_red[threadIdx.x * 8 + w];
+        col_scratch[(int64_t)threadIdx.x * XB_MAX_PARTIALS + blockIdx.x] = s;
+        __threadfence();
+    }
+    // statistics partials + arrival ticket (the __syncthreads inside block_sum_d orders the column stores above)
+    int *ticket = reinterpret_cast<int *>(scratch + 8 * XB_MAX_PARTIALS);
+    block_sum_d<6>(acc, red);
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int k = 0; k < 6; ++k) scratch[k * XB_MAX_PARTIALS + blockIdx.x] = acc[k];
+        __threadfence();
+        is_last = (atomicAdd(ticket, 1) == (int)gridDim.x - 1);
+    }
+    __syncthreads();
+    if (!is_last) return;
+    __threadfence();
+    const double d_ent = -(double)ent_coef * (double)B / (double)B_total;  // d(-ent_coef * mean_b H) / d log_std_d
+    for (int d = warp; d < D; d += nwarps) {
+        double s = 0.0;
+        for (int blk = lane; blk < (int)gridDim.x; blk += 32) s += __ldcg(&col_scratch[(int64_t)d * XB_MAX_PARTIALS + blk]);
+        s = warp_sum_d(s);
+        if (lane == 0) dlog_std[d] = (float)(s + d_ent);
+    }
+    double t[6] = {0, 0, 0, 0, 0, 0};
+    for (int blk = threadIdx.x; blk < (int)gridDim.x; blk += blockDim.x) {
+#pragma unroll
+        for (int k = 0; k < 6; ++k) t[k] += __ldcg(&scratch[k * XB_MAX_PARTIALS + blk]);
+    }
+    __syncthreads();
+    block_sum_d<6>(t, red);
+    if (threadIdx.x == 0) {
+        *ticket = 0;  // re-arm for the next launch
+        const double ib = (double)inv_bt;
+        float a_loss = (float)(t[0] * ib), c_loss = (float)(t[1] * ib), e = (float)(t[2] * ib);
+        stats[0] = a_loss;
+        stats[1] = c_loss;
+        stats[2] = e;
+        stats[3] = (float)(t[3] * ib);
+        stats[4] = (float)(t[4] * ib);
+        stats[5] = a_loss - ent_coef * e + vf_coef * c_loss;
+        stats[6] = 0.f;
+        stats[7] = 0.f;
+    }
+}
+
+extern "C" int xb_ppo_gaussian_loss_fwd_bwd(const float *mu, const float *log_std, const float *value,
+                                            const float *actions, const float *old_logp, const float *adv,
+                                            const float *ret, int64_t B, int D, int64_t B_total, float clip_range,
+                                            float vf_coef, float ent_coef, int loss_kind, float *dmu, float *dvalue,
+                                            float *dlog_std, float *stats, double *scratch, double *col_scratch,
+                                            void *stream) {
+    if (!mu || !log_std || !value || !actions || !adv || !ret || !dmu || !dvalue || !dlog_std || !stats || !scratch ||
+        !col_scratch)
+        return XB_EINVAL;
+    if (loss_kind != 0 && loss_kind != 1) return XB_EINVAL;
+    if (loss_kind == 0 && !old_logp) return XB_EINVAL;
+    if (B <= 0 || B_total < B || D <= 0) return XB_EINVAL;
+    if (D > 64) return XB_ERANGE;
+    cudaStream_t s = (cudaStream_t)stream;
+    int64_t want = (B + 255) / 256;
+    int grid = (int)(want < XB_MAX_PARTIALS ? want : XB_MAX_PARTIALS);
+    const float inv_bt = 1.0f / (float)B_total;
+#define XB_PPO_G(DM)                                                                                                  \
+    ppo_gaussian_loss_kernel<DM><<<grid, 256, 0, s>>>(mu, log_std, value, actions, old_logp, adv, ret, B, D, B_total, \
+                                                      inv_bt, clip_range, vf_coef, ent_coef, loss_kind, dmu, dvalue,  \
+                                                      dlog_std, stats, scratch, col_scratch)
+    if (D <= 8) XB_PPO_G(8);
+    else if (D <= 18) XB_PPO_G(18);
+    else if (D <= 32) XB_PPO_G(32);
+    else XB_PPO_G(64);
+#undef XB_PPO_G
+    return xb_launch_status();
+}
+
+// =====================================================================================================
 // K6  xb_dqn_td_fwd_bwd
 // =====================================================================================================
 __global__ void __launch_bounds__(256) dqn_td_kernel(const float *__restrict__ q_eval, const float *__restrict__ q_next,

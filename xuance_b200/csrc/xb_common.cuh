@@ -9,6 +9,7 @@
 #define XB_SM_COUNT_FALLBACK 148
 #define XB_MAX_PARTIALS 2048               // scratch doubles (per reduction slot group)
 #define XB_SCRATCH_DOUBLES (XB_MAX_PARTIALS * 8 + 8)
+#define XB_LOG_SQRT_2PI 0.91893853320467274178   // log(sqrt(2 pi)), the constant of Normal.log_prob
 
 static inline int xb_launch_status() {
     cudaError_t e = cudaPeekAtLastError();

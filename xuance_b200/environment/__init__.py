@@ -1,5 +1,5 @@
 """Environment construction (reference: xuance/environment/__init__.py:12-76 ``make_envs``)."""
-from .envs import REGISTRY_ENV, XuanCeEnvWrapper, CartPoleEnv, SyntheticAtariEnv
+from .envs import REGISTRY_ENV, XuanCeEnvWrapper, CartPoleEnv, SyntheticAtariEnv, SyntheticMuJoCoEnv
 from .ma_envs import SyntheticSMACEnv, XuanCeMultiAgentEnvWrapper
 from .vector_envs import (REGISTRY_VEC_ENV, VecEnv, DummyVecEnv, DummyVecEnv_Atari, SubprocVecEnv, SubprocVecEnv_Atari,
                           ShmSubprocVecEnv, ShmSubprocVecEnv_Atari, DummyVecMultiAgentEnv, SubprocVecMultiAgentEnv)

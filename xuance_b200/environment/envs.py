@@ -1,7 +1,8 @@
 """Raw environments available without third-party simulators (no gymnasium / ALE / SMAC in this image):
 ``CartPoleEnv`` - CartPole-v1 dynamics restated from the classic-control equations (BASELINE config 1 plumbing) -
 and ``SyntheticAtariEnv`` - Atari-SHAPED frames (84x84x4 uint8), sign-clipped rewards, rare terminals (the
-synthetic workload of BASELINE config 2; SURVEY.md section 8d).  ``XuanCeEnvWrapper`` adds the episode_step /
+synthetic workload of BASELINE config 2; SURVEY.md section 8d) - and ``SyntheticMuJoCoEnv`` - MuJoCo-SHAPED continuous
+control (17-d state, 6-d action in [-1, 1], HalfCheetah / Walker2d sizes) with a reward a policy can learn.  ``XuanCeEnvWrapper`` adds the episode_step /
 episode_score bookkeeping of xuance/environment/utils/wrapper.py:76-97 (actions are NOT rescaled: appendix B #17)."""
 import math
 
@@ -88,6 +89,45 @@ class SyntheticAtariEnv:
         return None
 
 
+class SyntheticMuJoCoEnv:
+    """Continuous-control stand-in of the MuJoCo shapes: observations are i.i.d. standard normal 17-vectors, the action is
+    clipped to the Box bounds, and the reward is -||a - W o||^2 for a FIXED matrix W (the same for every env and seed), so a
+    policy that learns the linear map o -> W o scores higher than the initial one.  Episodes end by truncation only."""
+    max_episode_steps = 100
+    obs_dim, act_dim = 17, 6
+
+    def __init__(self, seed=None):
+        self.observation_space = Box(-np.inf, np.inf, (self.obs_dim,), np.float32)
+        self.action_space = Box(-1.0, 1.0, (self.act_dim,), np.float32)
+        # target map: rows of norm ~0.5, so the best action 0.5 * N(0, 1) per dimension mostly lies inside the bounds
+        self.W = (np.random.default_rng(12345).normal(size=(self.act_dim, self.obs_dim)) * (0.5 / math.sqrt(self.obs_dim))
+                  ).astype(np.float32)
+        self.rng = np.random.default_rng(seed)
+        self.obs, self.steps = None, 0
+
+    def _observe(self):
+        self.obs = self.rng.normal(size=self.obs_dim).astype(np.float32)
+        return self.obs.copy()
+
+    def reset(self, seed=None, **kwargs):
+        if seed is not None:
+            self.rng = np.random.default_rng(seed)
+        self.steps = 0
+        return self._observe(), {}
+
+    def step(self, action):
+        a = np.clip(np.asarray(action, np.float32).reshape(self.act_dim), self.action_space.low, self.action_space.high)
+        reward = -float(np.square(a - self.W @ self.obs).sum())
+        self.steps += 1
+        return self._observe(), reward, False, self.steps >= self.max_episode_steps, {}
+
+    def close(self):
+        pass
+
+    def render(self, *a, **k):
+        return None
+
+
 class XuanCeEnvWrapper:
     def __init__(self, env, **kwargs):
         self.env = env
@@ -119,4 +159,4 @@ class XuanCeEnvWrapper:
         return self.env.close()
 
 
-REGISTRY_ENV = {"CartPole-v1": CartPoleEnv, "SyntheticAtari": SyntheticAtariEnv}
+REGISTRY_ENV = {"CartPole-v1": CartPoleEnv, "SyntheticAtari": SyntheticAtariEnv, "SyntheticMuJoCo": SyntheticMuJoCoEnv}

@@ -5,8 +5,8 @@ import numpy as np
 import torch
 
 from ...common.spaces import is_discrete, space2shape
-from ..utils.rollout_glue import categorical_act, DeviceRunningMeanStd, ActionReadback
-from ..rl_models import CategoricalActorHead, ValueHead, SharedActorCritic
+from ..utils.rollout_glue import categorical_act, gaussian_act, DeviceRunningMeanStd, ActionReadback
+from ..rl_models import CategoricalActorHead, GaussianActorHead, ValueHead, SharedActorCritic, ActivationFunctions
 from .on_policy import OnPolicyAgent
 
 
@@ -18,17 +18,19 @@ class PPO_Agent(OnPolicyAgent):
         self.learner = self._build_learner(self.config, self.model, self.callback)
 
     def _build_model(self):
-        """ppo_agent.py:40-93 (shared representation + categorical actor head + value head)."""
+        """ppo_agent.py:40-93 (shared representation + categorical or Gaussian actor head + value head)."""
         if not getattr(self.config, "shared_representation", True):
             raise NotImplementedError("separate actor/critic representations are outside the hot path scope")
         rep = self._build_representation(self.config.representation, self.observation_space, self.config)
-        if not is_discrete(self.action_space):
-            raise NotImplementedError("PPO with a Box action space (Gaussian head) is listed as 'next' in DESIGN.md; "
-                                      "the fused K4 loss covers the categorical policy of BASELINE configs 1-2")
         kw = dict(normalizer=self.normalize_fn, initializer=self.initializer, activation=self.activation,
                   device=self.device)
-        actor = CategoricalActorHead(feature_dim=rep.output_shapes['state'][0], hidden_size=self.config.actor_hidden_size,
-                                     action_dim=self.action_space.n, **kw)
+        if is_discrete(self.action_space):
+            actor = CategoricalActorHead(feature_dim=rep.output_shapes['state'][0],
+                                         hidden_size=self.config.actor_hidden_size, action_dim=self.action_space.n, **kw)
+        else:                                  # Box: tanh-style mu MLP + state-independent log_std (ppo_agent.py:54-57)
+            act_fn = ActivationFunctions[getattr(self.config, "activation_action", "tanh")]
+            actor = GaussianActorHead(feature_dim=rep.output_shapes['state'][0], hidden_size=self.config.actor_hidden_size,
+                                      action_dim=self.action_space.shape[0], activation_action=act_fn, **kw)
         critic = ValueHead(feature_dim=rep.output_shapes['state'][0], hidden_size=self.config.critic_hidden_size, **kw)
         return SharedActorCritic(representation=rep, actor=actor, critic=critic).to(self.device)
 
@@ -46,8 +48,10 @@ class PPO_Agent(OnPolicyAgent):
             shape = tuple(space2shape(self.observation_space))
             dt = torch.uint8 if np.dtype(getattr(self.observation_space, "dtype", np.float32)) == np.uint8 \
                 else torch.float32
+            rb = ActionReadback(self.n_envs, self.device) if is_discrete(self.action_space) else \
+                ActionReadback(self.n_envs, self.device, dtype=torch.float32, width=self.action_space.shape[0])
             self._dr = {"stage": torch.zeros((self.n_envs,) + shape, dtype=dt).pin_memory(),
-                        "readback": ActionReadback(self.n_envs, self.device),
+                        "readback": rb,
                         "rms": DeviceRunningMeanStd(shape, self.device) if self.use_obsnorm else None}
             if self.use_obsnorm:      # continue from whatever the host statistics hold (fresh, or a loaded checkpoint)
                 self._dr["rms"].load_state({'count': self.obs_rms.count, 'mean': self.obs_rms.mean,
@@ -86,13 +90,15 @@ class PPO_Agent(OnPolicyAgent):
         running-statistics + normalise, the network, K10 sample + log-prob written into the buffer's K1 staging rows,
         ONE read-back of N int32 actions, K1.  Episode bookkeeping (rewards, terminals, infos) stays on the host, where
         the environments live.  Random stream: torch's device generator (``torch.rand``) - the reference's
-        ``Categorical.sample`` stream cannot be reproduced by any fused kernel; distribution and log-prob are identical."""
+        ``Categorical.sample`` stream cannot be reproduced by any fused kernel; distribution and log-prob are identical.
+        A Gaussian policy takes K10-G with ``torch.randn`` noise instead and reads back N x D float32 actions."""
         dr = self._device_rollout_state()
         stage, rb, rms = dr["stage"], dr["readback"], dr["rms"]
         stage_np = stage.numpy()
         stage_np[...] = self.train_envs.buf_obs
         slots = self.memory.policy_slots()
         N = self.n_envs
+        gaussian = isinstance(self.model.actor, GaussianActorHead)
         train_info = {}
         for _ in range(train_steps):
             obs_d = stage.to(self.device, non_blocking=True)
@@ -100,10 +106,14 @@ class PPO_Agent(OnPolicyAgent):
             with torch.no_grad():
                 logits, values = self.model.forward_raw(obs_in)
                 slots["values"].copy_(values.reshape(N))
-                act = categorical_act(logits, uniforms=torch.rand(N, device=self.device), actions_f32=slots["actions"],
-                                      actions_i32=rb.dev, logp=slots["aux:old_logp"])
-            rb.launch()
-            acts = rb.wait().astype(np.int64)
+                if gaussian:
+                    act = gaussian_act(logits, self.model.actor.log_std, noise=torch.randn(logits.shape, device=self.device),
+                                       actions=slots["actions"], logp=slots["aux:old_logp"])
+                else:
+                    act = categorical_act(logits, uniforms=torch.rand(N, device=self.device), actions_f32=slots["actions"],
+                                          actions_i32=rb.dev, logp=slots["aux:old_logp"])
+            rb.launch(slots["actions"] if gaussian else None)
+            acts = rb.wait().copy() if gaussian else rb.wait().astype(np.int64)
             next_obs, rewards, terminals, truncations, infos = self.train_envs.step(acts)
             self.callback.on_train_step(self.current_step, envs=self.train_envs, policy=self.model, obs=obs_in,
                                         policy_out=act, acts=acts, vals=slots["values"], next_obs=next_obs,

@@ -2,8 +2,8 @@
 
 ``update(**samples)`` keeps the reference's signature, info keys and numerics (fp32 tolerance, tests/), but runs
 as: network forward (cuDNN/cuBLAS via torch) -> K4 fused loss forward+backward (one launch producing dlogits,
-dvalue and the logged statistics) -> torch backward through the network into the flat gradient bucket ->
-[one NCCL all-reduce] -> K7 fused clip-norm + Adam.  No ``.item()`` until the info dict is built (one D2H of
+dvalue and the logged statistics; K4-G for a Gaussian policy, which also produces dlog_std) -> torch backward through
+the network into the flat gradient bucket -> [one NCCL all-reduce] -> K7 fused clip-norm + Adam.  No ``.item()`` until the info dict is built (one D2H of
 8 floats; skipped entirely with ``sync=False`` as train_epochs does for all but the last minibatch)."""
 import torch
 
@@ -27,6 +27,14 @@ class PPO_Learner(Learner):
         self.clip_range = getattr(config, "clip_range", 0.0)
         self._stats = self.optimizer.bucket.tail[:8]      # the logged sums travel in the gradient bucket's tail
         self._scratch = _lib.scratch(self.device)
+        # a Gaussian policy (GaussianActorHead: mu + state-independent log_std) selects K4-G, which also needs room for the
+        # per-dimension partials of its log_std gradient
+        self._log_std = getattr(getattr(self.model, "actor", None), "log_std", None)
+        if self._log_std is not None:
+            n = _lib.load().xb_gaussian_scratch_doubles(self._log_std.numel())
+            if n <= 0:
+                raise ValueError("K4-G supports 1..64 action dimensions, the policy has %d" % self._log_std.numel())
+            self._col_scratch = torch.zeros(n, dtype=torch.float64, device=self.device)
         self._early = None
         self._hook_early_allreduce()
 
@@ -84,12 +92,22 @@ class PPO_Learner(Learner):
         dlogits = torch.empty_like(logits_c)
         dvalue = torch.empty_like(v_c)
         B_total = B * self.world_size
-        _lib.call("xb_ppo_loss_fwd_bwd", _lib.ptr(logits_c), _lib.ptr(v_c), _lib.ptr(act), _lib.ptr(old_logp),
-                  _lib.ptr(adv), _lib.ptr(ret), B, A, B_total, float(self.clip_range), float(self.vf_coef),
-                  float(self.ent_coef), self.loss_kind, _lib.ptr(dlogits), _lib.ptr(dvalue), _lib.ptr(self._stats),
-                  _lib.ptr(self._scratch))
-        self.optimizer.zero_grad()
-        torch.autograd.backward([logits_c, v_c], [dlogits, dvalue])
+        if self._log_std is None:
+            _lib.call("xb_ppo_loss_fwd_bwd", _lib.ptr(logits_c), _lib.ptr(v_c), _lib.ptr(act), _lib.ptr(old_logp),
+                      _lib.ptr(adv), _lib.ptr(ret), B, A, B_total, float(self.clip_range), float(self.vf_coef),
+                      float(self.ent_coef), self.loss_kind, _lib.ptr(dlogits), _lib.ptr(dvalue), _lib.ptr(self._stats),
+                      _lib.ptr(self._scratch))
+            self.optimizer.zero_grad()
+            torch.autograd.backward([logits_c, v_c], [dlogits, dvalue])
+        else:                                                # logits_c is the Gaussian mean mu [B, D], act [B, D]
+            log_std = self._log_std
+            dlog_std = torch.empty_like(log_std)
+            _lib.call("xb_ppo_gaussian_loss_fwd_bwd", _lib.ptr(logits_c), _lib.ptr(log_std), _lib.ptr(v_c), _lib.ptr(act),
+                      _lib.ptr(old_logp), _lib.ptr(adv), _lib.ptr(ret), B, A, B_total, float(self.clip_range),
+                      float(self.vf_coef), float(self.ent_coef), self.loss_kind, _lib.ptr(dlogits), _lib.ptr(dvalue),
+                      _lib.ptr(dlog_std), _lib.ptr(self._stats), _lib.ptr(self._scratch), _lib.ptr(self._col_scratch))
+            self.optimizer.zero_grad()
+            torch.autograd.backward([logits_c, v_c, log_std], [dlogits, dvalue, dlog_std])
         if self.world_size > 1:
             if self._early is not None:                      # the tail end of the bucket is already being reduced
                 off, work = self._early

@@ -42,9 +42,11 @@ class SharedActorCritic(nn.Module):
                            values=self.critic(rep_out.embeddings, **kwargs), rep_out=rep_out)
 
     def forward_raw(self, observation):
-        """(logits, values) without building a torch.distributions object - the fused K4 loss consumes these."""
+        """(logits, values) - or (mu, values) for a GaussianActorHead, whose log_std is ``self.actor.log_std`` - without
+        building a torch.distributions object: the fused K4 / K4-G losses and K10 / K10-G consume these."""
         z = self.representation(observation).embeddings
-        return self.actor.logits(z), self.critic(z)
+        head = self.actor.mu if isinstance(self.actor, GaussianActorHead) else self.actor.logits
+        return head(z), self.critic(z)
 
     def act(self, observation, deterministic=False, **kwargs):
         d = self.actor(self.representation(observation, **kwargs).embeddings, **kwargs)

@@ -4,9 +4,12 @@ the host, as single launches that leave their results in HBM.
 * ``categorical_act``        - K10: sample / argmax / log-prob / entropy of a categorical policy from raw logits
                                (``OnPolicyAgent.get_actions``, core/on_policy.py:128-169 +
                                ``CategoricalDistribution``, modules/distributions.py:128-162).
+* ``gaussian_act``           - K10-G: the same for a diagonal Gaussian policy from its mean and log-std
+                               (``DiagGaussianDistribution``, modules/distributions.py:165-197).
 * ``DeviceRunningMeanStd``   - K11: ``RunningMeanStd.update`` + ``Agent._process_observation``
                                (common/statistic_tools.py:117-185, agents/base/agent.py:262-279) on device arrays.
-* ``ActionReadback``         - the one device->host transfer a vector-env step needs: N int32 actions into pinned memory.
+* ``ActionReadback``         - the one device->host transfer a vector-env step needs: N int32 actions (or N x D float32
+                               continuous actions) into pinned memory.
 """
 import numpy as np
 import torch
@@ -44,6 +47,30 @@ def categorical_act(logits, uniforms=None, forced_actions=None, actions_f32=None
               _lib.ptr(actions_i32) if actions_i32 is not None else None, _lib.ptr(logp),
               _lib.ptr(entropy) if entropy is not None else None)
     return {"actions": actions_f32, "actions_i32": actions_i32, "logp": logp, "entropy": entropy, "_keep": keep}
+
+
+def gaussian_act(mu, log_std, noise=None, forced_actions=None, actions=None, logp=None, entropy=None):
+    """One K10-G launch over ``mu [N, D]`` and ``log_std [D]`` (float32, contiguous, CUDA).  Mode: ``forced_actions`` given ->
+    log-prob of those; else ``noise`` (standard normal [N, D]) given -> mu + noise * exp(log_std); else mu.  Output tensors
+    may be passed in (e.g. the rollout buffer's K1 staging); missing ones among (actions, logp) are allocated."""
+    if not mu.is_cuda:
+        raise RuntimeError("gaussian_act: mu must be a CUDA tensor (no CPU fallback)")
+    mu = mu.contiguous().float()
+    log_std = log_std.detach().contiguous().float()
+    N, D = mu.shape
+    if log_std.numel() != D:
+        raise ValueError("gaussian_act: log_std has %d entries for %d action dimensions" % (log_std.numel(), D))
+    if actions is None:
+        actions = torch.empty((N, D), dtype=torch.float32, device=mu.device)
+    if logp is None:
+        logp = torch.empty(N, dtype=torch.float32, device=mu.device)
+    keep = [mu, log_std]
+    for t in (noise, forced_actions):
+        if t is not None and (t.shape != mu.shape or t.dtype != torch.float32 or not t.is_contiguous()):
+            raise ValueError("gaussian_act: noise / forced_actions must be contiguous float32 [N, D] like mu")
+    _lib.call("xb_gaussian_act", _lib.ptr(mu), _lib.ptr(log_std), _lib.ptr(noise), _lib.ptr(forced_actions), N, D,
+              _lib.ptr(actions), _lib.ptr(logp), _lib.ptr(entropy))
+    return {"actions": actions, "logp": logp, "entropy": entropy, "_keep": keep}
 
 
 class DeviceRunningMeanStd:
@@ -104,17 +131,20 @@ class DeviceRunningMeanStd:
 
 class ActionReadback:
     """Double-buffered pinned block for the per-step actions: ``launch`` enqueues the D2H copy and records an event,
-    ``wait`` blocks on that event only (not on the whole device) and hands out the NumPy view."""
+    ``wait`` blocks on that event only (not on the whole device) and hands out the NumPy view.  Defaults: N int32
+    (discrete actions); ``dtype=torch.float32, width=D`` holds N x D continuous actions."""
 
-    def __init__(self, n_envs, device):
-        self.dev = torch.zeros(n_envs, dtype=torch.int32, device=device)
-        self.host = [torch.zeros(n_envs, dtype=torch.int32).pin_memory() for _ in range(2)]
+    def __init__(self, n_envs, device, dtype=torch.int32, width=None):
+        shape = (n_envs,) if width is None else (n_envs, width)
+        self.dev = torch.zeros(shape, dtype=dtype, device=device)
+        self.host = [torch.zeros(shape, dtype=dtype).pin_memory() for _ in range(2)]
         self.evt = [torch.cuda.Event(), torch.cuda.Event()]
         self.i = 0
 
-    def launch(self):
+    def launch(self, src=None):
+        """Copies ``src`` (a device tensor shaped like ``dev``, e.g. a buffer staging view the policy kernel wrote) or ``dev``."""
         self.i ^= 1
-        self.host[self.i].copy_(self.dev, non_blocking=True)
+        self.host[self.i].copy_(self.dev if src is None else src, non_blocking=True)
         self.evt[self.i].record()
 
     def wait(self):
